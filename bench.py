@@ -3,7 +3,7 @@
 WebQSP-shape synthetic subgraphs, with the aggregation kernel's achieved HBM bandwidth (roofline) and the
 CPU oracle port timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch: CSR batching of the fact list -> TypeLayer ->
@@ -14,6 +14,10 @@ pinned-host -> device copies, CSR batching, forward, ranking and the device -> h
 candidate lists, by wall clock between synchronizes.  Multi-GPU: one process per GPU, every rank runs its
 own B questions (weak scaling), no communication during the forward, one NCCL all-gather of the answer
 scores at the end of each step; time = max over ranks.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's questions) as DIR/<name>.npy, see
+dump_outputs().  Inputs and weights are seeded, so two builds run with the same arguments can be compared array by
+array.
 """
 import argparse
 import json
@@ -26,6 +30,7 @@ import time
 import numpy as np
 import torch
 
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -82,7 +87,14 @@ def parse():
                     help="0: dense-prior layers as aggregation kernel + GEMM instead of the fused layer kernel")
     ap.add_argument("--cuda-graph", type=int, default=1,
                     help="1: run the step through gnn_rag_b200.GraphedStep (CUDA-graph replay over static buffers)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (--impl ours)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def model_args_for(c, use_cuda):
@@ -177,7 +189,7 @@ def run_reference(a):
     default_nq = {"cfg3": 2, "cfg5": 1}.get(a.config, min(c["B"], 64))
     nq = min(a.cpu_sample if a.cpu_sample else default_nq, c["B"])
     heavy = a.config in ("cfg3", "cfg5")
-    steps = max(1, min(a.steps, 1 if heavy else 2))
+    steps = a.steps
     warmup = 0 if heavy else max(1, min(a.warmup, 1))
     qps, ms, cores, qps_l = cpu_oracle_run(c, sd, nq, steps, warmup)
     sample = "%d of %d questions per step, %d timed step(s), %d warm-up" % (nq, c["B"], steps, warmup)
@@ -248,6 +260,33 @@ def agg_algorithmic_bytes(B, N, F, D, I, R1, out_elem_bytes=4):
             + 2 * I * Nt * D * out_elem_bytes)
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, outs, limit=DUMP_LIMIT_BYTES):
+    """Write the step outputs ``outs`` ({name: tensor}, per-question arrays first in dim 0) to out_dir/<name>.npy:
+    floating point as float32, integers as float64 (exact).  ``cand_idx`` entries past ``cand_count`` are not part
+    of the result and are written as -1.  When the arrays would exceed ``limit`` bytes, a fixed seeded sample of
+    questions is written instead, and the sampled question indices go to question_rows.npy."""
+    host = {k: v.detach().cpu().numpy() for k, v in outs.items()}
+    idx = host["cand_idx"].copy()
+    idx[np.arange(idx.shape[1])[None, :] >= host["cand_count"][:, None]] = -1
+    host["cand_idx"] = idx
+    host = {k: v.astype(np.float32 if v.dtype.kind == "f" else np.float64) for k, v in host.items()}
+    B = host["pred_dist"].shape[0]
+    per_q = [k for k, v in host.items() if v.ndim and v.shape[0] == B]
+    row_bytes = sum(host[k][0].nbytes for k in per_q) + 8                 # + its entry in question_rows
+    fixed = sum(v.nbytes for k, v in host.items() if k not in per_q) + 128 * (len(host) + 1)   # + .npy headers
+    keep = (limit - fixed) // row_bytes
+    if keep < B:
+        rows = np.sort(np.random.RandomState(0).choice(B, int(keep), replace=False))
+        host = {k: (v[rows] if k in per_q else v) for k, v in host.items()}
+        host["question_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def run_ours(a):
     import torch.distributed as dist
 
@@ -295,12 +334,13 @@ def run_ours(a):
     gs = G.GraphedStep(model, S.WEBQSP_NUM_ENTITY) if a.cuda_graph else None
 
     def step_eager(batch):
-        _loss, _pred, pred_dist, _ = model(batch)
+        loss, pred, pred_dist, _ = model(batch)
         cand = ops.rank_candidates(pred_dist, model.last_batch.local_entity,
                                    model.last_batch.query_entities, S.WEBQSP_NUM_ENTITY, eps)
         if world > 1:
             parallel.all_gather_scores(pred_dist, B * world)
-        return pred_dist, cand
+        return dict(loss=loss, pred=pred, pred_dist=pred_dist, cand_idx=cand[0], cand_count=cand[1],
+                    cand_total=cand[2])
 
     def step(batch):
         if gs is None:
@@ -308,7 +348,8 @@ def run_ours(a):
         out = gs(batch)                     # copies the inputs into the static buffers, replays the graph
         if world > 1:
             parallel.all_gather_scores(out.pred_dist, B * world)
-        return out.pred_dist, out
+        return dict(loss=out.loss, pred=out.pred, pred_dist=out.pred_dist, cand_idx=out.cand_idx,
+                    cand_count=out.cand_count, cand_total=out.cand_total)
 
     def barrier():
         if world > 1:
@@ -371,7 +412,7 @@ def run_ours(a):
         flush.fill_(1)
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
-        step(dev_batch)
+        last = step(dev_batch)
         e.record()
         evs.append((s, e))
     barrier()
@@ -380,6 +421,8 @@ def run_ours(a):
     # clocks are sampled over the device-timed region only: nvidia-smi polling takes a driver lock and
     # perturbs the wall-clock e2e loop below (measured: 5.5 ms/step alone vs 8-19 ms with the sampler on)
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, last)     # before the e2e legs below replay the graph into the same buffers
     # ---- e2e: host (pinned) batch in, retrieved candidate lists out -------------------------------
     def e2e_step():
         if gs is None:

@@ -34,3 +34,11 @@ CASES = {   # name -> (loader kwargs, sample_ids, fact_dropout, numpy seed)
     "empty_questions": (dict(seed=4, num_questions=5, max_local_entity=6, num_kb_relation=4, facts_hi=1),
                         [0, 1, 2, 3, 4], 0.5, 14),
 }
+
+# Larger loader states (thousands of facts per batch), big enough for a meaningful timing comparison.
+LARGE_CASES = {
+    "large_a": (dict(seed=100, num_questions=12, max_local_entity=300, num_kb_relation=50, facts_lo=100, facts_hi=900),
+                list(np.random.RandomState(0).permutation(12)), 0.0, 7),
+    "large_b": (dict(seed=101, num_questions=20, max_local_entity=500, num_kb_relation=200, facts_lo=0, facts_hi=1500),
+                list(np.random.RandomState(1).permutation(20)), 0.25, 8),
+}

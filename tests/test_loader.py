@@ -1,7 +1,7 @@
 """CPU: gnn_rag_b200.loader.build_fact_mat is a bit-identical drop-in for the reference's
 BasicDataLoader._build_fact_mat (gnn/dataset_load.py:473-527) -- against golden outputs of the unmodified reference
-(tests/golden/loader/fact_mat_*.npz, made by tests/golden/make_fact_mat_golden.py) and, where the reference checkout is
-present, against the reference function itself on larger random loader states (with a timing comparison)."""
+(tests/golden/loader/fact_mat_*.npz, made by tests/golden/make_fact_mat_golden.py), including larger random loader
+states (with a timing comparison)."""
 import os
 import time
 
@@ -9,8 +9,7 @@ import numpy as np
 import pytest
 
 from gnn_rag_b200 import loader
-from loader_fixture import CASES, FakeLoader
-from oracle import ref_harness
+from loader_fixture import CASES, LARGE_CASES, FakeLoader
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "loader")
 KEYS = ("heads", "rels", "tails", "batch_ids", "fact_ids", "weight_list", "weight_rel_list")
@@ -122,23 +121,24 @@ def test_unshuffled_offset_concat_is_the_same_batch_up_to_fact_order():
         loader.build_fact_mat(ld, ids, 0.2, shuffle=False)
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference checkout not present")
-def test_build_fact_mat_matches_reference_live_and_is_faster():
-    ref_harness._import_reference()
-    import dataset_load                                          # the unmodified reference module
-    ref_fn = dataset_load.BasicDataLoader._build_fact_mat
-    for seed, (nq, nmax, nrel, lo, hi, dropout) in enumerate([(12, 300, 50, 100, 900, 0.0),
-                                                               (20, 500, 200, 0, 1500, 0.25)]):
-        ld = FakeLoader(seed=100 + seed, num_questions=nq, max_local_entity=nmax, num_kb_relation=nrel,
-                        facts_lo=lo, facts_hi=hi)
-        ids = list(np.random.RandomState(seed).permutation(nq))
-        np.random.seed(7 + seed)
+def test_build_fact_mat_matches_reference_golden_large_and_is_faster():
+    """Larger loader states: bit-identical to the reference's output (golden), and faster than the reference-form
+    restatement (oracle/loader_oracle.py), which is checked against the same golden."""
+    from oracle import loader_oracle
+    for name in sorted(LARGE_CASES):
+        kw, ids, dropout, seed = LARGE_CASES[name]
+        want = np.load(os.path.join(GOLD, "fact_mat_%s.npz" % name))
+        want = [want[k] for k in KEYS]
+        ld = FakeLoader(**kw)
+        np.random.seed(seed)
         t0 = time.perf_counter()
-        want = ref_fn(ld, ids, dropout)
+        ref_form = loader_oracle.build_fact_mat(ld, ids, dropout)
         t_ref = time.perf_counter() - t0
-        np.random.seed(7 + seed)
+        np.random.seed(seed)
         t0 = time.perf_counter()
         got = loader.build_fact_mat(ld, ids, dropout)
         t_new = time.perf_counter() - t0
+        assert got[0].dtype == np.int64
         assert_same(got, want)
-        assert t_new < t_ref, (t_new, t_ref)
+        assert_same(ref_form, want)
+        assert t_new < t_ref, (name, t_new, t_ref)
